@@ -9,6 +9,7 @@ dreamgaussian_b200/scene.py).
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            # our sm_100a path (the product)
   python bench.py --impl reference ...                           # the CPU oracle port, timed on the host cores
+  python bench.py ... --dump-outputs DIR                         # + the last timed step's gradients as DIR/*.npy
 
 One JSON line on stdout (rank 0).  See DESIGN.md "Measurement" for every field.
 """
@@ -36,6 +37,7 @@ WORKLOADS = {
     "cfg5": dict(points=2000000, res=1600, views_per_gpu=1, views=8, steps=100,
                  what="BASELINE.json configs[4]: 2M Gaussians, 1600x1600, SH degree 3, forward+backward, one view per GPU per step"),
 }
+DUMP_BYTES = 64 << 20          # --dump-outputs: cap on what one run writes
 
 
 def parse():
@@ -55,12 +57,34 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-rows", action="store_true", help="skip the short measurements of the SURVEY §8f rows (f1-f4)")
     ap.add_argument("--seed", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the per-Gaussian gradients of the last timed step as DIR/<name>.npy "
+                         "(float32; above %d MB in all, the same seeded sample of Gaussians from every array)" % (DUMP_BYTES >> 20))
     a = ap.parse_args()
     w = WORKLOADS[a.workload]
     for k in ("points", "res", "views_per_gpu", "views", "steps"):
         if getattr(a, k) is None:
             setattr(a, k, w[k])
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     return a
+
+
+def dump_outputs(out_dir, arrays, seed):
+    """arrays: name -> CUDA float32 tensor [P, ...], all with the same P.  Written whole when they fit DUMP_BYTES together,
+    else each restricted to the same rows: a sorted sample drawn from numpy's default_rng(seed), so that two builds dumped
+    with the same arguments hold the same Gaussians."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    P = next(iter(arrays.values())).shape[0]
+    row_bytes = sum(v[0].numel() * 4 for v in arrays.values()) if P else 0
+    rows = None
+    if P * row_bytes > DUMP_BYTES:
+        pick = np.sort(np.random.default_rng(seed).choice(P, DUMP_BYTES // row_bytes, replace=False))
+        rows = torch.tensor(pick, device=next(iter(arrays.values())).device)
+    for name, v in arrays.items():
+        x = v if rows is None else v.index_select(0, rows)
+        np.save(os.path.join(out_dir, name + ".npy"), x.float().cpu().numpy())
 
 
 def workload_name(a):
@@ -527,6 +551,9 @@ def run_ours(a, rank, world, local_rank):
     ms_total = float(ms_t.item())
     ms_per_step = ms_total / a.steps
     value = P * vpg * world * a.steps / (ms_total * 1e-3)
+    # what the last timed step handed back: the flat gradient (summed over this rank's views, all-reduced when N > 1)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, {"grad_" + k: v for k, v in vsr.grads.views.items() if v is not None}, a.seed)
 
     # ---------------- per-kernel CUDA-event timing (separate pass, same workload, this rank's stream) ----------------
     kern = {}
