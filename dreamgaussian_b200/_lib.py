@@ -68,6 +68,7 @@ EXPORTS = (
     "dgr_geom_bytes", "dgr_image_bytes", "dgr_binning_bytes",
     "dgr_forward_preprocess", "dgr_forward_render", "dgr_backward", "dgr_mark_visible", "dgr_debug_geom",
     "dgr_profile_enable", "dgr_profile_collect", "dgr_event_create", "dgr_event_synchronize", "dgr_event_destroy", "dgr_set_tuning", "dgr_peer_allreduce", "dgr_peer_flag_bytes", "dgr_peer_reduce_staged", "dgr_peer_push_flat", "dgr_knn_scratch_bytes", "dgr_dist_cuda2", "dgr_fields_scratch_bytes", "dgr_extract_fields", "dgr_adam_step", "dgr_densify_scratch_bytes", "dgr_densify_plan", "dgr_densify_apply",
+    "dgr_batch_geom_bytes", "dgr_batch_image_bytes", "dgr_forward_preprocess_batch", "dgr_backward_batch",
 )
 
 _lib = None
@@ -105,6 +106,14 @@ def load():
     lib.dgr_binning_bytes.argtypes = [u64, i32, i32]
     lib.dgr_forward_preprocess.restype = ctypes.c_int
     lib.dgr_forward_preprocess.argtypes = [ctypes.POINTER(DgrSettings), ctypes.POINTER(DgrGaussians), vp, vp, vp, vp]
+    lib.dgr_batch_geom_bytes.restype = ctypes.c_size_t
+    lib.dgr_batch_geom_bytes.argtypes = [i32, i32, i32, i32]
+    lib.dgr_batch_image_bytes.restype = ctypes.c_size_t
+    lib.dgr_batch_image_bytes.argtypes = [i32, i32, i32]
+    lib.dgr_forward_preprocess_batch.restype = ctypes.c_int        # settings: a ctypes array of V DgrSettings
+    lib.dgr_forward_preprocess_batch.argtypes = [vp, i32, ctypes.POINTER(DgrGaussians), vp, vp, vp, vp]
+    lib.dgr_backward_batch.restype = ctypes.c_int                  # settings / binning / capacities / gin: host arrays of V
+    lib.dgr_backward_batch.argtypes = [vp, i32, ctypes.POINTER(DgrGaussians), vp, vp, vp, vp, vp, vp, ctypes.POINTER(DgrGaussianGrads), vp]
     lib.dgr_peer_allreduce.restype = ctypes.c_int
     lib.dgr_peer_allreduce.argtypes = [vp, i32, i32, u64, u64, vp, ctypes.c_uint32, vp]
     lib.dgr_peer_reduce_staged.restype = ctypes.c_int

@@ -69,11 +69,12 @@ def is_stale():
 
 
 def build(force=False, verbose=False):
-    """Compile dreamgaussian_b200/csrc/dgr_api.cu -> dreamgaussian_b200/lib/libdgr_b200.so. Returns the path."""
+    """Compile dreamgaussian_b200/csrc/dgr_lib.cu (dgr_api.cu + the batched multi-view entry points) ->
+    dreamgaussian_b200/lib/libdgr_b200.so. Returns the path."""
     if not force and not is_stale():
         return LIB_PATH
     os.makedirs(LIB_DIR, exist_ok=True)
-    cmd = [_nvcc()] + NVCC_FLAGS + ["-o", LIB_PATH, os.path.join(CSRC, "dgr_api.cu")]
+    cmd = [_nvcc()] + NVCC_FLAGS + ["-o", LIB_PATH, os.path.join(CSRC, "dgr_lib.cu")]
     # the image's CC may point at a gcc without a usable spec dir; the system compiler is the host compiler
     if os.path.exists("/usr/bin/g++"):
         cmd += ["-ccbin", "/usr/bin/g++"]

@@ -107,3 +107,59 @@ def render_gaussian_model(gaussians, raster_settings, stats: Optional[DensifySta
         means2D=means2D, stats=stats)
     return {"image": color.clamp(0, 1), "depth": depth, "alpha": alpha, "viewspace_points": means2D,
             "visibility_filter": radii > 0, "radii": radii}
+
+
+class _RasterizeRawBatch(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, xyz, means2D, features_dc, features_rest, opacity_raw, scaling_raw, rotation_raw, settings_list, stats):
+        xyz = _r._dev_f32(xyz, "xyz")
+        dc = _r._dev_f32(features_dc, "features_dc")
+        rest = _r._opt(features_rest, "features_rest")
+        if rest is not None and rest.numel() == 0:
+            rest = None
+        op, sc, rot = _r._dev_f32(opacity_raw, "opacity"), _r._dev_f32(scaling_raw, "scaling"), _r._dev_f32(rotation_raw, "rotation")
+        color, radii, depth, alpha, state = _r.forward_batch_impl(settings_list, xyz, dc, op, sc, rot, sh_rest=rest, activations=True)
+        ctx.state, ctx.stats = state, stats
+        ctx.rest_shape = None if features_rest is None else tuple(features_rest.shape)
+        ctx.mark_non_differentiable(radii)
+        return color, radii, depth, alpha
+
+    @staticmethod
+    def backward(ctx, grad_color, grad_radii, grad_depth, grad_alpha):
+        state = ctx.state
+        # the statistics describe the RENDERS: a retain_graph / second backward must not count the views twice
+        stats = ctx.stats if not getattr(state, "stats_applied", False) else None
+        state.stats_applied = True
+        xyz, dc, op, sc, rot, rest = state.tensors
+        V, P = state.frame.V, state.frame.P
+        f32 = dict(dtype=torch.float32, device=xyz.device)
+        d_xyz, d_m2d = torch.empty((P, 3), **f32), torch.empty((V, P, 3), **f32)
+        d_dc = torch.empty((P, 1, 3), **f32)
+        d_rest = torch.empty(rest.shape, **f32) if rest is not None else None
+        d_op, d_sc, d_rot = torch.empty((P, 1), **f32), torch.empty((P, 3), **f32), torch.empty((P, 4), **f32)
+        _r.backward_batch_impl(state, *_r._batch_grads(state, grad_color, grad_depth, grad_alpha), d_xyz, d_m2d, d_dc, d_op, d_sc, d_rot,
+                               d_sh_rest=d_rest, densify=stats.as_tuple() if stats is not None else None)
+        if d_rest is None and ctx.rest_shape is not None:
+            d_rest = torch.zeros(ctx.rest_shape, **f32)
+        return d_xyz, d_m2d, d_dc, d_rest, d_op, d_sc, d_rot, None, None
+
+
+class BatchedFusedGaussianRasterizer(nn.Module):
+    """`BatchedGaussianRasterizer` for raw parameters: V views (1 to 16) of one GaussianModel in one call.
+    forward(xyz, features_dc, features_rest, opacity, scaling, rotation, means2D=None, stats=None) -> (color [V,3,H,W],
+    radii int32 [V,P], depth [V,1,H,W], alpha [V,1,H,W]).  Gradients of the raw tensors are summed over the views; means2D, when
+    given, is [V,P,3] and receives each view's screen-space gradient; `stats` (DensifyStats) is updated once per view, as V
+    single-view renders would update it."""
+
+    def __init__(self, settings_list):
+        super().__init__()
+        self.settings_list = _r.check_batch_settings(settings_list)
+
+    def forward(self, xyz, features_dc, features_rest, opacity, scaling, rotation, means2D: Optional[torch.Tensor] = None,
+                stats: Optional[DensifyStats] = None):
+        V = len(self.settings_list)
+        if means2D is None:
+            means2D = torch.zeros((V,) + tuple(xyz.shape), dtype=torch.float32, device=xyz.device, requires_grad=xyz.requires_grad)
+        elif tuple(means2D.shape) != (V,) + tuple(xyz.shape):
+            raise ValueError("means2D must have dimensions (num_views, num_points, 3)")
+        return _RasterizeRawBatch.apply(xyz, means2D, features_dc, features_rest, opacity, scaling, rotation, self.settings_list, stats)

@@ -343,3 +343,223 @@ class GaussianRasterizer(nn.Module):
             raise Exception("Please provide exactly one of either scale/rotation pair or precomputed 3D covariance!")
         return rasterize_gaussians(means3D, means2D, shs, colors_precomp, opacities, scales, rotations, cov3D_precomp,
                                    self.raster_settings)
+
+
+# ---------------------------------------------------------------------------------------------------------------------------------
+# Batched views: V cameras of ONE cloud at one resolution in one forward / backward (include/dgr_b200.h, "Batched views").  The
+# per-Gaussian stages run once for all views (inputs read once, summed gradient written once); binning, sort and both render
+# kernels run per view on that view's slice of the scratch.
+
+MAX_BATCH_VIEWS = 16
+_BATCH_SHARED = ("image_height", "image_width", "sh_degree", "scale_modifier", "prefiltered", "debug")
+
+
+def check_batch_settings(settings_list):
+    """The views of a batch share image size, SH degree, scale_modifier, prefiltered and debug; 1 to 16 views."""
+    settings_list = list(settings_list)
+    if not 1 <= len(settings_list) <= MAX_BATCH_VIEWS:
+        raise ValueError("a batch renders 1 to %d views, got %d" % (MAX_BATCH_VIEWS, len(settings_list)))
+    first = settings_list[0]
+    for i, rs in enumerate(settings_list[1:], 1):
+        for name in _BATCH_SHARED:
+            a, b = getattr(first, name), getattr(rs, name)
+            if (bool(a) != bool(b)) if name in ("prefiltered", "debug") else (a != b):
+                raise ValueError("view %d of the batch has %s = %r, view 0 has %r: the views of a batch must share %s"
+                                 % (i, name, b, a, ", ".join(_BATCH_SHARED)))
+    return settings_list
+
+
+def _reject_precomputed(colors_precomp, cov3D_precomp):
+    if colors_precomp is not None or cov3D_precomp is not None:
+        raise ValueError("the batched rasterizer takes SHs and scales / rotations: colors_precomp and cov3D_precomp are not supported")
+
+
+class _BatchFrame:
+    """ctypes views of one batched call's V settings + inputs (keeps the tensors alive)."""
+
+    def __init__(self, settings_list, means3D, sh, opacities, scales, rotations, sh_rest=None, activations=False):
+        self.frames = [_Frame(rs, means3D, sh, None, opacities, scales, rotations, None, sh_rest, activations) for rs in settings_list]
+        self.V = len(self.frames)
+        self.settings = (_lib.DgrSettings * self.V)(*[f.settings for f in self.frames])
+        self.gaussians = self.frames[0].gaussians
+        self.P, self.M = self.frames[0].P, self.frames[0].M
+
+
+_TICKET = [0]
+
+
+def _batch_counts(dev, V):
+    """Pinned (device-mapped) [16, 4] uint64 count slots, one row per view, per (host thread, device)."""
+    import threading
+    key = ("batch", threading.get_ident(), dev.index)
+    t = _SYNC.get(key)
+    if t is None:
+        t = torch.zeros((MAX_BATCH_VIEWS, 4), dtype=torch.int64).pin_memory()
+        _SYNC[key] = t
+    return t
+
+
+def _wait_tickets(counts, tickets, stream):
+    """Polls the ticket every view's scan kernel stores after its counts (no copy or event between the kernels)."""
+    arr = counts.numpy()
+    pending = list(range(len(tickets)))
+    spins = 0
+    while pending:
+        pending = [v for v in pending if int(arr[v, 2]) != tickets[v]]
+        spins += 1
+        if pending and spins % 2048 == 0 and stream.query():
+            pending = [v for v in pending if int(arr[v, 2]) != tickets[v]]
+            if pending:
+                raise RuntimeError("libdgr_b200: the instance counts of views %s never arrived" % pending)
+
+
+def forward_batch_impl(settings_list, means3D, sh, opacities, scales, rotations, sh_rest=None, activations=False):
+    """Both forward stages of V views.  Inputs are validated CUDA float32 tensors.  Returns (color [V,3,H,W], radii [V,P],
+    depth [V,1,H,W], alpha [V,1,H,W], BatchState).
+
+    Stage 1 is one batched call; then stage 2 of every view is enqueued with the shape's capacity hint before the host waits for
+    any instance count, and only a view whose guess was too small runs stage 2 again."""
+    lib = _lib.load()
+    dev = means3D.device
+    with torch.cuda.device(dev):
+        fr = _BatchFrame(settings_list, means3D, sh, opacities, scales, rotations, sh_rest, activations)
+        V, P = fr.V, fr.P
+        H, W = int(settings_list[0].image_height), int(settings_list[0].image_width)
+        u8 = dict(dtype=torch.uint8, device=dev)
+        color = torch.empty((V, 3, H, W), dtype=torch.float32, device=dev)
+        depth = torch.empty((V, 1, H, W), dtype=torch.float32, device=dev)
+        alpha = torch.empty((V, 1, H, W), dtype=torch.float32, device=dev)
+        radii = torch.empty((V, P), dtype=torch.int32, device=dev)
+        geom_stride, image_stride = lib.dgr_geom_bytes(P, H, W), lib.dgr_image_bytes(H, W)
+        geom = torch.empty((lib.dgr_batch_geom_bytes(V, P, H, W),), **u8)
+        image = torch.empty((lib.dgr_batch_image_bytes(V, H, W),), **u8)
+        st = _stream_ptr(dev)
+        _lib.check(lib.dgr_forward_preprocess_batch(fr.settings, V, ctypes.byref(fr.gaussians), _ptr(geom), _ptr(image), _ptr(radii), st))
+        hint = get_capacity_hint(dev.index, P, H, W)
+        cap0, big0 = hint if hint is not None else (max(65536, 16 * P), True)
+        caps, bigs, binnings, outs = [cap0] * V, [bool(big0)] * V, [None] * V, [None] * V
+        counts = _batch_counts(dev, V)
+        cnt_base = counts.data_ptr()
+
+        def stage2(v, flags, ticket, event=None):
+            binnings[v] = torch.empty((lib.dgr_binning_bytes(caps[v], H, W),), **u8)
+            outs[v] = _lib.DgrImages(_ptr(color[v]), _ptr(depth[v]), _ptr(alpha[v]), _ptr(radii[v]))
+            _lib.check(lib.dgr_forward_render(ctypes.byref(fr.settings[v]), ctypes.byref(fr.gaussians),
+                                              ctypes.c_void_p(geom.data_ptr() + v * geom_stride), _ptr(binnings[v]), ctypes.c_uint64(caps[v]),
+                                              ctypes.c_void_p(image.data_ptr() + v * image_stride), ctypes.byref(outs[v]),
+                                              (1 if bigs[v] else 0) | flags, ctypes.c_void_p(cnt_base + 32 * v), ctypes.c_uint64(ticket),
+                                              event, st))
+
+        tickets = []
+        for v in range(V):
+            _TICKET[0] += 1
+            tickets.append(_TICKET[0])
+            stage2(v, 0, tickets[v])
+        _wait_tickets(counts, tickets, torch.cuda.current_stream(dev))
+        n_inst = [int(counts[v, 0]) for v in range(V)]
+        n_big = [int(counts[v, 1]) for v in range(V)]
+        for v in range(V):
+            while n_inst[v] > caps[v] or (n_big[v] > 0 and not bigs[v]):       # this view's guess was wrong: redo its stage 2 (rare)
+                caps[v] = max(caps[v], int(n_inst[v] * 1.25) + 4096)
+                bigs[v] = bigs[v] or n_big[v] > 0
+                event = _host_sync_objects(dev)[1]
+                stage2(v, 2, 0, event)                                         # DGR_FLAG_RERUN; counts copied into row v, then the event
+                _lib.check(lib.dgr_event_synchronize(event))
+                n_inst[v], n_big[v] = int(counts[v, 0]), int(counts[v, 1])
+        set_capacity_hint(dev.index, P, H, W, max(max(int(n * 1.25) + 4096 for n in n_inst), 65536), any(b > 0 for b in n_big))
+    state = BatchState()
+    state.frame, state.geom, state.image, state.binnings, state.capacities = fr, geom, image, binnings, caps
+    state.radii, state.num_rendered = radii, n_inst
+    state.tensors = (means3D, sh, opacities, scales, rotations, sh_rest)
+    return color, radii, depth, alpha, state
+
+
+class BatchState:
+    """What a batched forward leaves behind for its backward: V scratch slices, V binning buffers and their capacities."""
+    __slots__ = ("frame", "geom", "image", "binnings", "capacities", "radii", "num_rendered", "tensors", "stats_applied")
+
+
+def backward_batch_impl(state, grad_color, grad_depth, grad_alpha, d_means3D, d_means2D, d_sh, d_opac, d_scales, d_rot,
+                        accumulate=False, d_sh_rest=None, densify=None):
+    """The backward of a batched forward: per-view upstream gradients [V, ...] (any may be None = zeros) in; means3D / shs (/ shs_rest)
+    / opacities / scales / rotations gradients summed over the views written (or added with accumulate) into the given tensors;
+    d_means2D is [V, P, 3].  densify = (xyz_gradient_accum, denom, max_radii2D), updated once per view."""
+    lib = _lib.load()
+    fr = state.frame
+    V = fr.V
+    dev = state.radii.device
+    with torch.cuda.device(dev):
+        view = lambda t, v: None if t is None else ctypes.c_void_p(t[v].data_ptr())
+        gin = (_lib.DgrImageGrads * V)(*[_lib.DgrImageGrads(view(grad_color, v), view(grad_depth, v), view(grad_alpha, v)) for v in range(V)])
+        binning = (ctypes.c_void_p * V)(*[b.data_ptr() for b in state.binnings])
+        caps = (ctypes.c_uint64 * V)(*state.capacities)
+        gout = _lib.DgrGaussianGrads(_ptr(d_means3D), _ptr(d_means2D), _ptr(d_sh), None, _ptr(d_opac), _ptr(d_scales), _ptr(d_rot), None,
+                                     1 if accumulate else 0, _ptr(d_sh_rest),
+                                     *((_ptr(t) for t in densify) if densify is not None else (None, None, None)), None)
+        _lib.check(lib.dgr_backward_batch(fr.settings, V, ctypes.byref(fr.gaussians), _ptr(state.geom), binning, caps, _ptr(state.image),
+                                          _ptr(state.radii), gin, ctypes.byref(gout), _stream_ptr(dev)))
+
+
+def _batch_upstream(g, name, shape):
+    if g is None:
+        return None
+    g = _dev_f32(g, name)
+    if tuple(g.shape) != tuple(shape):
+        raise ValueError("%s must have shape %s" % (name, tuple(shape)))
+    return g
+
+
+class _RasterizeBatch(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, means3D, means2D, sh, opacities, scales, rotations, settings_list):
+        means3D, opacities = _dev_f32(means3D, "means3D"), _dev_f32(opacities, "opacities")
+        sh, scales, rotations = _dev_f32(sh, "shs"), _dev_f32(scales, "scales"), _dev_f32(rotations, "rotations")
+        color, radii, depth, alpha, state = forward_batch_impl(settings_list, means3D, sh, opacities, scales, rotations)
+        ctx.state = state
+        ctx.mark_non_differentiable(radii)
+        return color, radii, depth, alpha
+
+    @staticmethod
+    def backward(ctx, grad_color, grad_radii, grad_depth, grad_alpha):
+        state = ctx.state
+        means3D, sh, opacities, scales, rotations, _ = state.tensors
+        V, P = state.frame.V, state.frame.P
+        f32 = dict(dtype=torch.float32, device=means3D.device)
+        d_means3D, d_means2D = torch.empty((P, 3), **f32), torch.empty((V, P, 3), **f32)
+        d_sh, d_opac = torch.empty(sh.shape, **f32), torch.empty((P, 1), **f32)
+        d_scales, d_rot = torch.empty((P, 3), **f32), torch.empty((P, 4), **f32)
+        backward_batch_impl(state, *_batch_grads(state, grad_color, grad_depth, grad_alpha), d_means3D, d_means2D, d_sh, d_opac, d_scales, d_rot)
+        # ctx.state stays: a retain_graph backward runs again from the same buffers (they go away with the graph node)
+        return d_means3D, d_means2D, d_sh, d_opac, d_scales, d_rot, None
+
+
+def _batch_grads(state, grad_color, grad_depth, grad_alpha):
+    s = state.frame.frames[0].settings
+    V, H, W = state.frame.V, int(s.image_height), int(s.image_width)
+    return (_batch_upstream(grad_color, "grad_color", (V, 3, H, W)), _batch_upstream(grad_depth, "grad_depth", (V, 1, H, W)),
+            _batch_upstream(grad_alpha, "grad_alpha", (V, 1, H, W)))
+
+
+class BatchedGaussianRasterizer(nn.Module):
+    """V views (1 to 16) of one cloud in one call.  The views share image size, SH degree, scale_modifier, prefiltered and
+    debug; fov, bg, view / projection matrices and camera position may differ.
+
+    forward(means3D, opacities, shs, scales, rotations, means2D=None) -> (color [V,3,H,W], radii int32 [V,P], depth [V,1,H,W],
+    alpha [V,1,H,W]).  The gradients of means3D / shs / opacities / scales / rotations are summed over the views; means2D, when
+    given, is the [V,P,3] per-view screen-space dummy whose .grad receives each view's own gradient."""
+
+    def __init__(self, settings_list):
+        super().__init__()
+        self.settings_list = check_batch_settings(settings_list)
+
+    def forward(self, means3D, opacities, shs, scales, rotations, means2D=None, colors_precomp=None, cov3D_precomp=None):
+        _reject_precomputed(colors_precomp, cov3D_precomp)
+        if shs is None or scales is None or rotations is None:
+            raise ValueError("the batched rasterizer needs shs, scales and rotations")
+        V = len(self.settings_list)
+        if means2D is None:
+            means2D = torch.zeros((V,) + tuple(means3D.shape), dtype=torch.float32, device=means3D.device,
+                                  requires_grad=means3D.requires_grad)
+        elif tuple(means2D.shape) != (V,) + tuple(means3D.shape):
+            raise ValueError("means2D must have dimensions (num_views, num_points, 3)")
+        return _RasterizeBatch.apply(means3D, means2D, shs, opacities, scales, rotations, self.settings_list)

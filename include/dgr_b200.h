@@ -174,6 +174,32 @@ int dgr_backward(const DgrSettings *s, const DgrGaussians *g, void *geom, const 
                  uint64_t capacity_instances, const void *image, const int32_t *radii, const float *out_alpha,
                  const DgrImageGrads *gin, const DgrGaussianGrads *gout, void *stream);
 
+/* == Batched views: V cameras (1 <= V <= 16) of ONE cloud at ONE resolution ==
+ * A batch gives what V single-view calls give when their backwards accumulate into the same gradient buffers, but the
+ * per-Gaussian stages read the inputs once for all views and write the summed gradient once.
+ *   - s is a HOST array of V DgrSettings.  image_height / image_width, sh_degree, scale_modifier, prefiltered and debug must be
+ *     equal in all of them; tanfovx / tanfovy, bg, viewmatrix, projmatrix and campos may differ.
+ *   - g: SHs (plain or raw, DgrGaussians.activations) and scales / rotations; colors_precomp / cov3D_precomp are rejected.
+ *     Every per-Gaussian input pointer must be 16-byte aligned (misaligned input is rejected).
+ *   - Scratch: ONE geom allocation of dgr_batch_geom_bytes(V, P, H, W) and ONE image allocation of dgr_batch_image_bytes(V, H, W);
+ *     view v's geom scratch starts at geom + v * dgr_geom_bytes(P, H, W) and its image scratch at image + v * dgr_image_bytes(H, W)
+ *     (both strides are multiples of 256 bytes; the base pointers are 256-byte aligned).  Each view has its own binning buffer.
+ *   - radii is [V, P] int32 (view v at radii + v * P).
+ * dgr_forward_preprocess_batch leaves in every view's scratch exactly what dgr_forward_preprocess leaves there for that view; stage
+ * 2 of view v is then dgr_forward_render(&s[v], g, view v's geom, view v's binning, ..., view v's image, ...) as for one view.
+ * dgr_backward_batch runs the backward render of every view (binning[v] / capacity[v]: HOST arrays, the buffers and capacities
+ * stage 2 of view v ran with) and then ONE per-Gaussian backward over all views.  gin is a HOST array of V DgrImageGrads.  gout:
+ * means3D / shs (/ shs_rest) / opacities / scales / rotations gradients summed over the views (written, or added with accumulate);
+ * dL_dmeans2D is [V, P, 3], per view; xyz_gradient_accum / denom / max_radii2D are updated once per view with radii > 0, as V
+ * single-view backwards do; dL_dcolors_precomp / dL_dcov3D_precomp are unused and push must be NULL. */
+size_t dgr_batch_geom_bytes(int32_t num_views, int32_t P, int32_t image_height, int32_t image_width);
+size_t dgr_batch_image_bytes(int32_t num_views, int32_t image_height, int32_t image_width);
+int dgr_forward_preprocess_batch(const DgrSettings *s, int32_t num_views, const DgrGaussians *g, void *geom, void *image,
+                                 int32_t *radii, void *stream);
+int dgr_backward_batch(const DgrSettings *s, int32_t num_views, const DgrGaussians *g, void *geom, void *const *binning,
+                       const uint64_t *capacity_instances, const void *image, const int32_t *radii, const DgrImageGrads *gin,
+                       const DgrGaussianGrads *gout, void *stream);
+
 /* Multi-GPU (view-sharded data parallelism, SURVEY.md §8e): all-reduce(sum) of the flat float32 gradient buffer over
  * NVLink with this library's own kernel.  The buffer lives in symmetric memory: peer_ptrs[w] (HOST array of `world` device
  * addresses) is rank w's copy mapped into this process; multicast_ptr, if non-zero, is the NVSwitch multicast address of
